@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- BASELINE.json metric on synthetic data.
 
-python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the front-end hot path over one batch (128 per GPU) of synthetic
 1280x720 frames (BASELINE.json configs[1]: 8 levels, 2000 features): per frame
@@ -19,6 +19,9 @@ nothing on this path: weak scaling, no data-path collective.
           synthetic config-4 graph (N=1) / config-5 graph sharded by landmark
           with one NCCL all-reduce per trial (N>1)
   roofline / cpu_baseline : see DESIGN.md "Measurement"
+
+--dump-outputs DIR writes what the last timed step handed back on rank 0 (keypoints, descriptors, match
+assignments; see dump_outputs) as DIR/<name>.npy, so that two builds can be compared on identical inputs.
 """
 import argparse
 import ctypes as C
@@ -506,6 +509,42 @@ class Workload:
         return h2d, d2h
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(wl, step, out_dir):
+    """Write what step `step` of the device-resident loop handed back, per frame of its batch: the keypoints and
+    descriptors of the extraction, the assignments and match counts of both projection matchers.  Per-keypoint
+    arrays are the frames' rows one after the other (keypoints_per_frame gives the split).  Integers and bytes are
+    stored as float32, which holds them exactly.  A batch whose outputs could exceed DUMP_BYTES is represented by a
+    fixed (seed 0) sample of its frames, listed in frames.npy."""
+    p = step % wl.POOL
+    e = wl.meta[p]
+    per_frame = wl.cap * (6 + 32 + 2) * 4 + 5 * 4
+    max_frames = (DUMP_BYTES - 4096) // per_frame   # 4096: the .npy headers
+    frames = np.arange(wl.B)
+    if wl.B > max_frames:
+        frames = np.sort(np.random.default_rng(0).choice(wl.B, max_frames, replace=False))
+    assign_last = wl.d_assign_last.cpu().numpy()
+    assign_local = wl.d_assign_local.cpu().numpy()
+    kps, desc, mono, n_kp, a_last, a_local = [], [], [], [], [], []
+    for b in frames:
+        m, k, d = wl.ext.download_results(int(b))
+        mono.append(m)
+        n_kp.append(len(k))
+        kps.append(np.stack([k[f].astype(np.float32) for f in ("x", "y", "size", "angle", "response", "octave")], 1))
+        desc.append(d.astype(np.float32))
+        a_last.append(assign_last[b, :e["n"][b]])     # the matchers' frame views hold e["n"][b] keypoints
+        a_local.append(assign_local[b, :e["n"][b]])
+    out = {"frames": frames, "mono_index": mono, "keypoints_per_frame": n_kp,
+           "keypoints": np.concatenate(kps), "descriptors": np.concatenate(desc),
+           "assign_last": np.concatenate(a_last), "assign_local": np.concatenate(a_local),
+           "matches_last": wl.nmatch_last[frames], "matches_local": wl.nmatch_local[frames]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32))
+
+
 def run_lba_gpu(rank, world, device):
     """LocalBA on the GPU: configs 4 and 5 at N=1, config 5 sharded by landmark for N>1 (one ncclAllReduce of the
     envelope of [S | b_s] per LM trial).  `value` = LM trials / device time of optimize(10); `e2e` = the same count
@@ -867,7 +906,12 @@ def main():
     ap.add_argument("--no-lba", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-stereo", action="store_true", help="skip the 8(f) legs (ComputeStereoMatches, PoseOptimization, isInFrustum, ComputeBoW)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -936,6 +980,8 @@ def main():
     ms_dev = e0.elapsed_time(e1)
     launches = launches_now() - launches0
     nm_last, nm_local = int(wl.nmatch_last.sum()), int(wl.nmatch_local.sum())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl, K - 1, args.dump_outputs)
     # ---- end to end through the host-buffer ABI (wall clock brackets every copy and sync).
     # Batches come from independent camera streams, so `--e2e-workers` host threads (each with its
     # own extractor + matcher handles, i.e. its own CUDA streams) work on different batches at once:
