@@ -10,9 +10,9 @@
 // host -- the analogue of g2o's buildStructure (block_solver.hpp:143-295).
 //
 // Kernels per LM trial:
-//   lin_kernel          residuals, Huber weights, Jacobians, H_ll, b_l, W (6x3 per edge)
+//   lin_edge_kernel     residuals, Huber weights, Jacobians, W (6x3 per edge); lm_gather_kernel sums H_ll, b_l
 //   pose_reduce_kernel  H_pp, b_p per free pose (fixed-order tree sum)
-//   lm_prepare_kernel   (H_ll + lambda I)^-1, D^-1 b_l, Y = W D^-1
+//   lm_prepare_kernel   (H_ll + lambda I)^-1, D^-1 b_l; y_edge_kernel Y = W D^-1
 //   schur_pairs_kernel  S_{i1 i2} = [H_pp] - sum_l Y_{i1 l} W_{i2 l}^T : the dense contraction,
 //                       on the tensor cores as fp64 DMMA (mma.sync.m8n8k4.f64), one CTA per pose pair
 //   bschur_kernel       b_s = b_p - sum W D^-1 b_l          (stored as an extra row of S)
@@ -20,7 +20,7 @@
 //   ldlt_kernel         blocked right-looking LDL^T of S (+rhs row), all SMs, own grid barrier
 //   backsub_kernel      L^T x_p = z
 //   lm_update_kernel    x_l = D^-1 (b_l - W^T x_p), state backup, oplus (SE3 exp), scale terms
-//   err_kernel          robust chi2 of the trial state
+//   chi_kernel          robust chi2 of the trial state
 // The LM control law (lambda, rho, accept/reject, stop rules) runs on the host
 // between trials, reading three doubles back per trial; *stop is polled there.
 #include <cuda_runtime.h>
@@ -289,24 +289,22 @@ __device__ __forceinline__ void store_pose_records(const LbaDev& D, int e, const
   for (int i = 0; i < 9; i++) We2[i] = make_double2(we[2 * i], we[2 * i + 1]);
 }
 
-// One thread per landmark: all its edges (base_binary_edge.hpp:55-120).  LINEARIZE = false evaluates the robust chi2 of
-// a trial state; the linearising pass runs one thread per EDGE instead (lin_edge_kernel + lm_gather_kernel below) unless
-// ORB_B200_LIN=landmark.
-template <bool LINEARIZE, bool RIG>
-__global__ void __launch_bounds__(128) lin_kernel(LbaDev D) {
+// Robust chi2 of a trial state, one thread per landmark: all its edges (base_binary_edge.hpp:55-120).  The
+// linearising pass runs one thread per EDGE instead (lin_edge_kernel + lm_gather_kernel below).
+template <bool RIG>
+__global__ void __launch_bounds__(128) chi_kernel(LbaDev D) {
   const int l = blockIdx.x * 128 + threadIdx.x;
   if (l >= D.n_mp) return;
   const double X[3] = {D.pts[3 * (size_t)l], D.pts[3 * (size_t)l + 1], D.pts[3 * (size_t)l + 2]};
-  double Hl[6] = {0, 0, 0, 0, 0, 0}, bl[3] = {0, 0, 0}, chi = 0;
+  double chi = 0;
   // the keyframe index -> pose hop is two dependent global loads: the pose of the NEXT edge is fetched while this
-  // edge is linearised (ncu: long-scoreboard stalls were 60 % of all samples at 16 warps per SM)
+  // edge is evaluated (ncu: long-scoreboard stalls were 60 % of all samples at 16 warps per SM)
   const int e_begin = D.lm_ptr[l], e_end = D.lm_ptr[l + 1];
   int k_next = e_begin < e_end ? D.e_kf[e_begin] : 0;
   double Pn[7];
 #pragma unroll
   for (int c = 0; c < 7; c++) Pn[c] = D.pose[7 * (size_t)k_next + c];
   for (int e = e_begin; e < e_end; e++) {
-    const int k = k_next;
     double P[7];
 #pragma unroll
     for (int c = 0; c < 7; c++) P[c] = Pn[c];
@@ -324,36 +322,11 @@ __global__ void __launch_bounds__(128) lin_kernel(LbaDev D) {
     double rho0, rho1;
     robustify(D.e_stereo[e] == LBA_EDGE_STEREO ? D.hs : D.hm, e2, rho0, rho1);  // body edges: thHuberMono (:1380-1382)
     chi += rho0;
-    if (!LINEARIZE) continue;
-    double A[9], B[18];
-    edge_jacobians<RIG>(D, e, k, q, P, Xc, A, B);
-    const double s = (double)D.e_is2[e];
-    const double ws = rho1 * s;
-    double orr[3];
-#pragma unroll
-    for (int i = 0; i < 3; i++) orr[i] = -(s * r[i]) * rho1;
-    // landmark block (upper: 00 01 02 11 12 22)
-    int t = 0;
-#pragma unroll
-    for (int i = 0; i < 3; i++) {
-#pragma unroll
-      for (int j = i; j < 3; j++) {
-        Hl[t++] += ws * (A[i] * A[j] + A[3 + i] * A[3 + j] + A[6 + i] * A[6 + j]);
-      }
-      bl[i] += A[i] * orr[0] + A[3 + i] * orr[1] + A[6 + i] * orr[2];
-    }
-    if (D.e_free[e] >= 0) store_pose_records(D, e, A, B, ws, orr);
   }
   D.chi_lm[l] = chi;
-  if (LINEARIZE) {
-    double* H = D.Hll + 6 * (size_t)l;
-#pragma unroll
-    for (int i = 0; i < 6; i++) H[i] = Hl[i];
-    D.bl[3 * (size_t)l] = bl[0]; D.bl[3 * (size_t)l + 1] = bl[1]; D.bl[3 * (size_t)l + 2] = bl[2];
-  }
 }
 
-// The linearising pass, one thread per EDGE: a landmark has ~6.5 edges, so the thread-per-landmark kernel above runs
+// The linearising pass, one thread per EDGE: a landmark has ~6.5 edges, so a thread per landmark (as in chi_kernel) runs
 // 6.5 x fewer threads, each a serial loop of dependent loads (edge -> keyframe -> pose) -- ncu: 12 % of the DRAM
 // throughput, 13 % of the issue slots.  Here every edge is its own thread; its contribution to the landmark block
 // (H_ll upper triangle, b_l, robust chi2: 10 doubles) goes to a per-edge record that lm_gather_kernel adds up per
@@ -501,9 +474,7 @@ __global__ void __launch_bounds__(1024) maxdiag_kernel(LbaDev D, const double* H
   if (threadIdx.x == 0) { for (int w = 0; w < 32; w++) m = fmax(m, sm[w]); *out = m; }
 }
 
-// Per landmark: D^-1 = (H_ll + lambda I)^-1 (cofactors), D^-1 b_l; WITH_Y: also Y_e = W_e D^-1 of its edges
-// (ORB_B200_LIN=landmark); otherwise y_edge_kernel forms Y one thread per edge.
-template <bool WITH_Y>
+// Per landmark: D^-1 = (H_ll + lambda I)^-1 (cofactors), D^-1 b_l; y_edge_kernel then forms Y one thread per edge.
 __global__ void __launch_bounds__(128) lm_prepare_kernel(LbaDev D, double lambda) {
   const int l = blockIdx.x * 128 + threadIdx.x;
   if (l >= D.n_mp) return;
@@ -521,25 +492,10 @@ __global__ void __launch_bounds__(128) lm_prepare_kernel(LbaDev D, double lambda
   const double* b = D.bl + 3 * (size_t)l;
 #pragma unroll
   for (int i = 0; i < 3; i++) D.db[3 * (size_t)l + i] = Di[i * 3] * b[0] + Di[i * 3 + 1] * b[1] + Di[i * 3 + 2] * b[2];
-  if (!WITH_Y) return;
-  for (int e = D.lm_ptr[l]; e < D.lm_ptr[l + 1]; e++) {
-    if (D.e_free[e] < 0) continue;
-    // 144-byte records, 16-byte aligned: nine 16-byte loads / stores instead of eighteen 8-byte ones
-    const double2* We2 = reinterpret_cast<const double2*>(D.W + 18 * (size_t)e);
-    double2* Ye2 = reinterpret_cast<double2*>(D.Y + 18 * (size_t)e);
-    double We[18], Ye[18];
-#pragma unroll
-    for (int i = 0; i < 9; i++) { const double2 v = We2[i]; We[2 * i] = v.x; We[2 * i + 1] = v.y; }
-#pragma unroll
-    for (int i = 0; i < 6; i++)
-#pragma unroll
-      for (int j = 0; j < 3; j++) Ye[i * 3 + j] = We[i * 3] * Di[j] + We[i * 3 + 1] * Di[3 + j] + We[i * 3 + 2] * Di[6 + j];
-#pragma unroll
-    for (int i = 0; i < 9; i++) Ye2[i] = make_double2(Ye[2 * i], Ye[2 * i + 1]);
-  }
 }
 
 // Y_e = W_e D_l^-1, one thread per edge (the edges of a landmark are neighbours: its D^-1 comes from L1 / L2).
+// 144-byte records, 16-byte aligned: nine 16-byte loads / stores instead of eighteen 8-byte ones.
 __global__ void __launch_bounds__(128) y_edge_kernel(LbaDev D) {
   const int e = blockIdx.x * 128 + threadIdx.x;
   if (e >= D.n_edges || D.e_free[e] < 0) return;
@@ -670,7 +626,7 @@ __device__ __forceinline__ void grid_barrier(unsigned* bar, unsigned nblocks, un
   __syncthreads();
 }
 
-__global__ void __launch_bounds__(256) ldlt_kernel(double* __restrict__ M, int n, unsigned* bar, double* fail, int dbg) {
+__global__ void __launch_bounds__(256) ldlt_kernel(double* __restrict__ M, int n, unsigned* bar, double* fail) {
   __shared__ double L11[NB][NB + 1];
   __shared__ double Dd[NB];
   __shared__ double Ti[NB][NB + 1];
@@ -686,7 +642,7 @@ __global__ void __launch_bounds__(256) ldlt_kernel(double* __restrict__ M, int n
       L11[r][c] = (r < nb && c <= r) ? M[(size_t)(k0 + r) * n + k0 + c] : 0.0;
     }
     __syncthreads();
-    if (threadIdx.x < 32 && !(dbg & 1)) {
+    if (threadIdx.x < 32) {
       // right-looking LDL^T of the 32x32 block by one warp: lane r keeps row r in registers, the
       // scaled column is broadcast through shared memory.  The serial chain per column is one
       // reciprocal + one FMA (the left-looking form chained a whole dot product: 12.8 us / panel).
@@ -727,7 +683,7 @@ __global__ void __launch_bounds__(256) ldlt_kernel(double* __restrict__ M, int n
     const int r0 = k0 + nb;
     {
       const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-      for (int i = r0 + blockIdx.x * 8 + warp; i < rows && !(dbg & 2); i += 8 * nblk) {
+      for (int i = r0 + blockIdx.x * 8 + warp; i < rows; i += 8 * nblk) {
         double* Mi = M + (size_t)i * n + k0;
         double a = (lane < nb) ? Mi[lane] : 0.0;
         for (int m = 0; m < nb; m++) {
@@ -749,7 +705,7 @@ __global__ void __launch_bounds__(256) ldlt_kernel(double* __restrict__ M, int n
     // ---- trailing update, 32x32 tiles (bi >= bj), rhs row is the last partial tile row
     const int T = (rows - r0 + NB - 1) / NB;
     const int ntiles = T * (T + 1) / 2;
-    for (int tile = blockIdx.x; tile < ntiles && !(dbg & 4); tile += nblk) {
+    for (int tile = blockIdx.x; tile < ntiles; tile += nblk) {
       // tile -> (bi, bj), bi >= bj
       int bi = (int)((sqrt(8.0 * tile + 1.0) - 1.0) * 0.5);
       while ((bi + 1) * (bi + 2) / 2 <= tile) bi++;
@@ -981,9 +937,9 @@ __global__ void __launch_bounds__(SKY_THREADS) ldlt_sky_kernel(double* __restric
 // rows enter it once, from global memory, when the envelope first reaches them (independent loads, off the
 // critical path), are updated in place panel after panel, and leave as finished columns of L.  Panels are 8
 // columns wide: the 8x8 pivot block is factored by one thread entirely in registers (no communication on the
-// chain), the panel rows by one thread each, the rank-8 update of the window in 4x4 register micro-tiles;
-// three barriers per 8 pivots instead of 64 per 32.  The back-substitution runs in the same launch, 8 unknowns
-// per step, with the next step's rows of L already in flight.
+// chain), the panel rows on the tensor pipe through the inverse of the pivot block, the rank-8 update of the window
+// in 8x8 DMMA tiles; two barriers per 8 pivots instead of 64 per 32.  The back-substitution runs in the same launch,
+// 8 unknowns per step, with the next step's rows of L already in flight.
 constexpr int WIN = 128, WIN_P = WIN + 1, WIN_ROWS = WIN - 8, WPB = 8, WIN_THREADS = 512;
 constexpr int WIN_LP = 132;  // row pitch of the m-major L / L*D panels: the four k-rows of a DMMA fragment fall into different banks
 
@@ -1003,10 +959,6 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 __device__ __forceinline__ int wmod(int v) { return v & (WIN - 1); }  // v % WIN for v >= 0 (ring indices)
 static_assert((WIN & (WIN - 1)) == 0, "ring size must be a power of two");
 
-// PROF (ORB_B200_LDLT_PROF): cycle counters of the phases as seen by warp 0, printed by lba_solve
-__device__ unsigned long long g_win_prof[32];
-static int win_prof_solves = 0;
-
 // One side of a solve: the matrix (its own (n+1) x n buffer), its envelope tables, and -- for the two-sided solve --
 // where the side stops.  WinArgs.mode: 0 = factor everything and back-substitute (one CTA, side 0);
 // 1 = factor panels [0, pend) and write the window that is left (the separator rows with this side's Schur
@@ -1019,20 +971,19 @@ struct WinSide {
 struct WinArgs {
   WinSide s[2];
   double* fail; double* x; const double* xs;
-  int flags, mode, msep;  // msep: first separator column in the caller's numbering (side 1 runs in reversed numbering)
+  int mode, msep;  // msep: first separator column in the caller's numbering (side 1 runs in reversed numbering)
 };
 
-template <bool PROF, bool FWD_MMA>
-__global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa) {
+// __grid_constant__: wa.s[blockIdx.x] is read in place from the parameter space; without it the compiler may copy
+// the whole struct to local memory to index it
+__global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const __grid_constant__ WinArgs wa) {
   const WinSide& sd = wa.s[blockIdx.x];
   double* __restrict__ M = sd.M;
-  const int n = sd.n, flags = wa.flags, mode = wa.mode;
+  const int n = sd.n, mode = wa.mode;
   const int* __restrict__ reach = sd.reach;
   const int* __restrict__ first_g = sd.first;
   double* fail = wa.fail;
   double* __restrict__ x = wa.x;
-  // flags (experiments, ORB_B200_LDLT_FLAGS): bit 0 = equal tile shares for all 15 tile warps (measured +2 %), bit 1 =
-  // generic three-at-a-time tile loop update_run3 (measured +7 %), bit 2 = reversed warp numbering for the roles
   extern __shared__ __align__(16) double win_dyn[];
   double* A = win_dyn;                       // [WIN][WIN_P] ring of the trailing window
   double* zr = A + WIN * WIN_P;              // [WIN] right-hand side entries of the window columns
@@ -1045,20 +996,9 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
   __shared__ double Dib[WPB];                // 1 / D
   __shared__ double Gi[WPB][WPB];            // inverse of the unit lower-triangular pivot block (phase (A) on the tensor pipe)
   __shared__ unsigned short tile_ij[(WIN / 8) * (WIN / 8 + 1) / 2];  // lower-triangle tile number -> (ti << 8) | tj
-  // flags bit 2 numbers the warps against the hardware's order (a scheduler picks the eligible warp with the highest
-  // hardware id first, so the pivot warp would be served first): measured, no difference (4.06 vs 4.07 ms).
   const int lane = threadIdx.x & 31;
-  const int warp = (flags & 4) ? (WIN_THREADS / 32 - 1) - (int)(threadIdx.x >> 5) : (int)(threadIdx.x >> 5), tid = warp * 32 + lane;
+  const int warp = (int)(threadIdx.x >> 5), tid = warp * 32 + lane;
   const int npan = (n + WPB - 1) / WPB;
-  unsigned long long pc[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  long long t0 = 0;
-  auto tick = [&](int slot) {
-    if (PROF) {
-      long long t;
-      asm volatile("mov.u64 %0, %%clock64;" : "=l"(t) :: "memory");
-      pc[slot] += (unsigned long long)(t - t0); t0 = t;
-    }
-  };
   for (int i = tid; i < n; i += WIN_THREADS) first[i] = first_g[i];
   for (int p = tid; p < npan; p += WIN_THREADS) {
     const int k0 = p * WPB, nb = min(WPB, n - k0);
@@ -1128,7 +1068,7 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
   };
   // G = L_bb^-1 (unit lower triangular) after pivot(): lane r of the pivot's warp forms column r,
   // g[c] = -sum_{m<c} L[c][m] g[m] below the diagonal (L[c][c] = 1), one uniform instruction stream for the eight
-  // lanes.  Phase (A) multiplies the panel rows by G^T on the tensor pipe instead of substituting one thread per row.
+  // lanes.  Phase (A) multiplies the panel rows by G^T on the tensor pipe.
   auto pivot_inverse = [&]() {
     __syncwarp();
     if (lane < WPB) {
@@ -1209,40 +1149,6 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
       }
     }
   };
-  // FWD_MMA build: every tile through one path, three at a time with all operand loads first.  A warp runs this as
-  // one dependent instruction stream (one eligible warp per scheduler issues every ~4 cycles), so what counts is the
-  // number of instructions per tile, not their latency: tile coordinates come from the table, the predicates are the
-  // only per-tile branches, and nothing is carried from tile to tile.
-  auto update_run3 = [&](int t_begin, int t_end, int r0, int nr) {
-    constexpr int G = 3;
-    const int acol = ft * WIN_LP + fg, ccol = r0 + 2 * ft;
-    for (int t = t_begin; t < t_end; t += G) {
-      int i0[G], i1[G];
-      bool ok0[G], ok1[G];
-      double a0[G], a1[G], b0[G], b1[G], c0[G], c1[G];
-#pragma unroll
-      for (int u = 0; u < G; u++) {
-        const bool live = t + u < t_end;
-        const int tt = tile_ij[min(t + u, t_end - 1)];
-        const int ti8 = (tt >> 8) * 8, tj8 = (tt & 255) * 8;
-        const int wi = ti8 + fg, wj = tj8 + 2 * ft;
-        a0[u] = -Lt[acol + ti8]; a1[u] = -Lt[acol + 4 * WIN_LP + ti8];
-        b0[u] = LDt[acol + tj8]; b1[u] = LDt[acol + 4 * WIN_LP + tj8];
-        const int rowoff = (wi >= nr) ? ZR_OFF : wmod(r0 + wi) * WIN_P;  // the rhs row has no column of its own
-        ok0[u] = live && wi <= nr && wj < nr && wj <= wi;
-        ok1[u] = live && wi <= nr && wj + 1 < nr && wj + 1 <= wi;
-        i0[u] = rowoff + wmod(ccol + tj8); i1[u] = rowoff + wmod(ccol + tj8 + 1);
-        c0[u] = ok0[u] ? A[i0[u]] : 0.0; c1[u] = ok1[u] ? A[i1[u]] : 0.0;
-      }
-#pragma unroll
-      for (int u = 0; u < G; u++) mma2(c0[u], c1[u], a0[u], a1[u], b0[u], b1[u]);
-#pragma unroll
-      for (int u = 0; u < G; u++) {
-        if (ok0[u]) A[i0[u]] = c0[u];
-        if (ok1[u]) A[i1[u]] = c1[u];
-      }
-    }
-  };
   // the tile of the next pivot block, on the critical path: no tile bookkeeping at all
   auto update_tile0 = [&](int r0, int nr) {
     const int wj = 2 * ft;
@@ -1257,8 +1163,8 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
     if (ok0) A[i0] = c0;
     if (ok1) A[i1] = c1;
   };
-  // warps of phase (A): one thread per panel row (WIN / 32 warps hold a whole window), or -- on the tensor pipe --
-  // four 8-row blocks per warp; the other warps bring rows into the window
+  // warps of phase (A): four 8-row blocks per warp (WIN / 32 warps cover a whole window); the other warps bring rows
+  // into the window
   // (measured: eight forward warps + eight loaders is 6 % slower than four + twelve -- 4.06 vs 3.81 ms per optimize(10)
   // at config 5 -- although phase (A) itself gets shorter)
   constexpr int FWD_WARPS = WIN / 32;
@@ -1310,11 +1216,10 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
     __syncthreads();
     if (warp == 0) {
       if (tid == 0) pivot(0);
-      if (FWD_MMA) pivot_inverse();
+      pivot_inverse();
     }
   }
   __syncthreads();
-  if (PROF) asm volatile("mov.u64 %0, %%clock64;" : "=l"(t0) :: "memory");
   for (int p = 0; p < pend; p++) {
     const int k0 = p * WPB, nb = min(WPB, n - k0);
     const int R = rlast[p];  // last row of the window; rows [k0, R] are resident, the pivot block is factored
@@ -1322,68 +1227,44 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
     // rows of the next pivot block that are not resident yet (narrow or ending envelope) are loaded by warp 0 in (B)
     const int r0 = k0 + nb, nr = R - r0 + 1;  // nr rows under the pivot block; slot nr = rhs
     const int pre = more ? min(r0 + WPB - 1, n - 1) : R;
-    // ---- (A) panel rows [k0+nb, R] and the rhs row: forward substitution, one thread per row.  The other warps
+    // ---- (A) panel rows [k0+nb, R] and the rhs row: forward substitution on the tensor pipe.  The other warps
     //      bring in the rows the NEXT panel adds to the window (their ring slots are free: the window of panel p+1
     //      starts at r0), so the global-memory latency is off the chain.
-    if (FWD_MMA) {
-      // (L*D) rows = A_rows * L_bb^-T: one 8-row block per warp trip, two fp64 DMMA m8n8k4 (A[g][t] = window row
-      // g, panel column t / t+4; B[t][g] = G[g][t] / G[g][t+4]; C[g][2t], C[g][2t+1]); L = (L*D) / D.  The rhs row
-      // is row nr of the window (zr).  Blocks of a warp are independent: all operand loads first.
-      if (warp < FWD_WARPS) {
-        const int nblk = (nr + 1 + 7) >> 3;
-        const double g0 = Gi[fg][ft], g1 = Gi[fg][ft + 4];
-        const double di0 = Dib[2 * ft], di1 = Dib[2 * ft + 1];
-        constexpr int FB = (WIN / 8 + FWD_WARPS - 1) / FWD_WARPS;  // row blocks per forward warp
-        double a0[FB], a1[FB], c0[FB], c1[FB];
+    // (L*D) rows = A_rows * L_bb^-T: one 8-row block per warp trip, two fp64 DMMA m8n8k4 (A[g][t] = window row
+    // g, panel column t / t+4; B[t][g] = G[g][t] / G[g][t+4]; C[g][2t], C[g][2t+1]); L = (L*D) / D.  The rhs row
+    // is row nr of the window (zr).  Blocks of a warp are independent: all operand loads first.
+    if (warp < FWD_WARPS) {
+      const int nblk = (nr + 1 + 7) >> 3;
+      const double g0 = Gi[fg][ft], g1 = Gi[fg][ft + 4];
+      const double di0 = Dib[2 * ft], di1 = Dib[2 * ft + 1];
+      constexpr int FB = (WIN / 8 + FWD_WARPS - 1) / FWD_WARPS;  // row blocks per forward warp
+      double a0[FB], a1[FB], c0[FB], c1[FB];
 #pragma unroll
-        for (int u = 0; u < FB; u++) {
-          const int wi = 8 * (warp + u * FWD_WARPS) + fg;
-          const bool valid = warp + u * FWD_WARPS < nblk && wi <= nr;
-          const int rowoff = (wi >= nr) ? ZR_OFF : (wmod(r0 + wi)) * WIN_P;
-          a0[u] = (valid && ft < nb) ? A[rowoff + wmod(k0 + ft)] : 0.0;
-          a1[u] = (valid && ft + 4 < nb) ? A[rowoff + wmod(k0 + ft + 4)] : 0.0;
-          c0[u] = 0.0; c1[u] = 0.0;
-        }
+      for (int u = 0; u < FB; u++) {
+        const int wi = 8 * (warp + u * FWD_WARPS) + fg;
+        const bool valid = warp + u * FWD_WARPS < nblk && wi <= nr;
+        const int rowoff = (wi >= nr) ? ZR_OFF : (wmod(r0 + wi)) * WIN_P;
+        a0[u] = (valid && ft < nb) ? A[rowoff + wmod(k0 + ft)] : 0.0;
+        a1[u] = (valid && ft + 4 < nb) ? A[rowoff + wmod(k0 + ft + 4)] : 0.0;
+        c0[u] = 0.0; c1[u] = 0.0;
+      }
 #pragma unroll
-        for (int u = 0; u < FB; u++)
-          if (warp + u * FWD_WARPS < nblk) mma2(c0[u], c1[u], a0[u], a1[u], g0, g1);
+      for (int u = 0; u < FB; u++)
+        if (warp + u * FWD_WARPS < nblk) mma2(c0[u], c1[u], a0[u], a1[u], g0, g1);
 #pragma unroll
-        for (int u = 0; u < FB; u++) {
-          if (warp + u * FWD_WARPS >= nblk) continue;
-          const int wi = 8 * (warp + u * FWD_WARPS) + fg;
-          const double l0 = c0[u] * di0, l1 = c1[u] * di1;   // columns >= nb: c = 0 (a = 0 there and G is triangular)
-          Lt[(2 * ft) * WIN_LP + wi] = l0; Lt[(2 * ft + 1) * WIN_LP + wi] = l1;
-          LDt[(2 * ft) * WIN_LP + wi] = c0[u]; LDt[(2 * ft + 1) * WIN_LP + wi] = c1[u];
-          if (wi <= nr) {
-            double* dst = M + (size_t)(wi == nr ? n : r0 + wi) * n + k0 + 2 * ft;
-            if (2 * ft + 1 < nb) *reinterpret_cast<double2*>(dst) = make_double2(l0, l1);  // n even, k0 % 8 == 0: 16-byte aligned
-            else if (2 * ft < nb) dst[0] = l0;
-          }
+      for (int u = 0; u < FB; u++) {
+        if (warp + u * FWD_WARPS >= nblk) continue;
+        const int wi = 8 * (warp + u * FWD_WARPS) + fg;
+        const double l0 = c0[u] * di0, l1 = c1[u] * di1;   // columns >= nb: c = 0 (a = 0 there and G is triangular)
+        Lt[(2 * ft) * WIN_LP + wi] = l0; Lt[(2 * ft + 1) * WIN_LP + wi] = l1;
+        LDt[(2 * ft) * WIN_LP + wi] = c0[u]; LDt[(2 * ft + 1) * WIN_LP + wi] = c1[u];
+        if (wi <= nr) {
+          double* dst = M + (size_t)(wi == nr ? n : r0 + wi) * n + k0 + 2 * ft;
+          if (2 * ft + 1 < nb) *reinterpret_cast<double2*>(dst) = make_double2(l0, l1);  // n even, k0 % 8 == 0: 16-byte aligned
+          else if (2 * ft < nb) dst[0] = l0;
         }
       }
-    } else if (tid <= nr) {
-      const bool rhs = tid == nr;
-      const int i = r0 + tid;
-      double* src = rhs ? zr : A + (wmod(i)) * WIN_P;
-      double ld[WPB], l[WPB];
-#pragma unroll
-      for (int m = 0; m < WPB; m++) ld[m] = m < nb ? src[wmod(k0 + m)] : 0.0;
-#pragma unroll
-      for (int m = 1; m < WPB; m++)
-#pragma unroll
-        for (int p2 = 0; p2 < m; p2++) ld[m] -= ld[p2] * Lb[m][p2];
-#pragma unroll
-      for (int m = 0; m < WPB; m++) {
-        l[m] = m < nb ? ld[m] * Dib[m] : 0.0;
-        Lt[m * WIN_LP + tid] = l[m];
-        LDt[m * WIN_LP + tid] = m < nb ? ld[m] : 0.0;
-      }
-      double* dst = M + (size_t)(rhs ? n : i) * n + k0;
-#pragma unroll
-      for (int m = 0; m < WPB; m++)
-        if (m < nb) dst[m] = l[m];
     }
-    tick(0);
     if (warp >= FWD_WARPS) {
       commit_row();  // the row of panel p+1 fetched one panel ago
       if (warp == FWD_WARPS) pivot_store(p);
@@ -1396,9 +1277,7 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
         }
       }
     }
-    tick(5);
     __syncthreads();
-    tick(1);
     // ---- (B) rank-nb update of the window on the tensor pipe, with look-ahead: warp 0 updates the tile that
     //      holds the NEXT pivot block first and then factors it (one thread) while the other warps update the
     //      rest of the window
@@ -1411,30 +1290,18 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
         if (pre > R) load_rows(R + 1, pre, r0, 0, 1);
         update_tile0(r0, nr);
         __syncwarp();
-        tick(2);
         if (tid == 0 && more) pivot(p + 1);
-        if (FWD_MMA && more) pivot_inverse();
-        tick(6);
-      } else if (FWD_MMA && (flags & 1)) {
-        // equal shares: the pivot warp's chain (tile, 8 reciprocals, inverse) is longer than any share
-        const int per = (ntile - 1 + 14) / 15;
-        const int tb = 1 + (warp - 1) * per;
-        if (flags & 2) update_run3(min(tb, ntile), min(tb + per, ntile), r0, nr);
-        else update_run(min(tb, ntile), min(tb + per, ntile), r0, nr);
-        tick(2);
+        if (more) pivot_inverse();
       } else {
         const int T = ntile - 1;
         const int light = T / 22, heavy = (T - 3 * light + 11) / 12;
         int tb, te;
         if (warp & 3) { tb = 1 + (warp - 1 - (warp >> 2)) * heavy; te = tb + heavy; }
         else { const int rest = max(T - 12 * heavy, 0), per = (rest + 2) / 3; tb = 1 + 12 * heavy + ((warp >> 2) - 1) * per; te = tb + per; }
-        if (FWD_MMA && (flags & 2)) update_run3(min(tb, ntile), min(te, ntile), r0, nr);
-        else update_run(min(tb, ntile), min(te, ntile), r0, nr);
-        tick(2);
+        update_run(min(tb, ntile), min(te, ntile), r0, nr);
       }
     }
     __syncthreads();
-    tick(3);
   }
   // ---- L^T x = z (z = row n of M, already scaled by 1/D), 8 unknowns per step, four warps, one named barrier per
   //      step.  With G = L_bb^-T (the inverse of the step's unit-triangular pivot block) the step is
@@ -1494,7 +1361,6 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
     jmb[bq] = jmv;  // (after the reads of `first`: jmb may alias nothing, it lives in the ring)
   }
   __syncthreads();
-  tick(8);
   constexpr int BS_THREADS = WIN;  // one thread per window column (WIN_ROWS < WIN)
   if (tid < BS_THREADS) {
     double Pc[WPB];
@@ -1531,7 +1397,6 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
     cp_async_wait<1>();
     transform(b0);
     if (b0 > 1) fetch(b0 - 2); else cp_async_commit();
-    tick(13);
     for (int bq = b0; bq >= 0; bq--) {
       const int k0 = bq * WPB;
       const int j = jmb[bq] + tid;
@@ -1544,23 +1409,18 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
         const double s1 = Pc[4] * ab[4] + Pc[5] * ab[5] + Pc[6] * ab[6] + Pc[7] * ab[7];
         acc[j] -= s0 + s1;
       }
-      tick(9);
       // ---- off the chain: the next step's row of P (its rows arrived two steps ago), the copies of the step after
       //      the next.  One group is committed per step so that wait_group counts steps.
       if (bq > 0) {
         cp_async_wait<1>();
         transform(bq - 1);
-        tick(10);
         if (bq > 2) fetch(bq - 3); else cp_async_commit();
-        tick(11);
       }
       asm volatile("bar.sync 1, %0;" ::"n"(BS_THREADS) : "memory");
-      tick(12);
     }
     cp_async_wait<0>();
   }
   __syncthreads();
-  tick(14);
   // x_b = G acc_b for every block at once: G[r][c] = Linv[c][r] (c > r), 1 on the diagonal
   for (int i = tid; i < ksep; i += WIN_THREADS) {
     const int bq = i / WPB, r = i - bq * WPB, k0 = bq * WPB, nb = min(WPB, n - k0);
@@ -1571,14 +1431,6 @@ __global__ void __launch_bounds__(WIN_THREADS) ldlt_win_kernel(const WinArgs wa)
   }
   if (mode == 2 && blockIdx.x == 0)
     for (int i = ksep + tid; i < esep; i += WIN_THREADS) x[i] = wa.xs[i - ksep];
-  if (PROF) {
-    tick(4);
-    if (tid == 0 || tid == 32)
-      for (int k = 0; k < 8; k++) atomicAdd(&g_win_prof[(tid ? 8 : 0) + k], pc[k]);
-    if (tid == 0) {  // back-substitution in detail; slot 4 is then only the x pass
-      for (int k = 8; k < 16; k++) atomicAdd(&g_win_prof[8 + k], pc[k]);
-    }
-  }
 }
 
 // ---- two-sided reduced solve ("burn at both ends")
@@ -1968,7 +1820,7 @@ static int solve_impl(Solver& S, const lba_graph_view* g, const volatile uint8_t
     lm_ptr[g->e_mp[e] + 1]++;
   }
   // rig extension of the view: KannalaBrandt8 cameras and / or second-camera (EdgeSE3ProjectXYZToBody) edges take the
-  // general-camera instantiation of lin_kernel; plain Pinhole windows keep the specialised one
+  // general-camera instantiations of the edge kernels; plain Pinhole windows keep the specialised ones
   bool any_kb8 = false;
   for (int k = 0; k < K && g->kf_cam_model; k++) any_kb8 |= g->kf_cam_model[k] == ORB_CAM_KB8;
   if (any_kb8 && !g->kf_cam_dist) { set_last_error("lba_solve: kf_cam_model names a KannalaBrandt8 camera but kf_cam_dist is NULL"); return ORB_E_ARG; }
@@ -2043,7 +1895,7 @@ static int solve_impl(Solver& S, const lba_graph_view* g, const volatile uint8_t
   // pattern; the natural order is kept when it is at least as good (what Eigen's AMD ordering does for g2o).
   std::vector<int> pos(nf);  // pos[natural free index] = free index used from here on
   for (int i = 0; i < nf; i++) pos[i] = i;
-  if (nf > 2 && !getenv("ORB_B200_LBA_NO_REORDER")) {
+  if (nf > 2) {
     auto profile = [&](const std::vector<int>& q) {  // q[f] = position of pose f
       long long p = 0;
       std::vector<int> lo(nf);
@@ -2381,18 +2233,15 @@ static int solve_impl(Solver& S, const lba_graph_view* g, const volatile uint8_t
   };
   // chi (robust) of the current state -> h_scalars[0]; all ranks see the global value
   auto eval_chi = [&](bool linearize) -> int {
+    // rig: KannalaBrandt8 cameras / second-camera edges take the general-camera instantiations
     if (L) {
-      static const bool lin_by_landmark = getenv("ORB_B200_LIN") && !strcmp(getenv("ORB_B200_LIN"), "landmark");
-      if (linearize && !lin_by_landmark) {  // one thread per edge + a per-landmark gather
+      if (linearize) {  // one thread per edge + a per-landmark gather
         if (rig) lin_edge_kernel<true><<<(E + 127) / 128, 128, 0, st>>>(D, d_lmc);
         else lin_edge_kernel<false><<<(E + 127) / 128, 128, 0, st>>>(D, d_lmc);
         lm_gather_kernel<<<lm_blocks, 128, 0, st>>>(D, d_lmc);
         S.launches += 1;
-      } else if (rig) {  // KannalaBrandt8 cameras / second-camera edges: the general-camera instantiation
-        if (linearize) lin_kernel<true, true><<<lm_blocks, 128, 0, st>>>(D);
-        else lin_kernel<false, true><<<lm_blocks, 128, 0, st>>>(D);
-      } else if (linearize) lin_kernel<true, false><<<lm_blocks, 128, 0, st>>>(D);
-      else lin_kernel<false, false><<<lm_blocks, 128, 0, st>>>(D);
+      } else if (rig) chi_kernel<true><<<lm_blocks, 128, 0, st>>>(D);
+      else chi_kernel<false><<<lm_blocks, 128, 0, st>>>(D);
     }
     reduce_kernel<<<1, 1024, 0, st>>>(D.chi_lm, L, D.scalars);
     S.launches += 2;
@@ -2454,14 +2303,10 @@ static int solve_impl(Solver& S, const lba_graph_view* g, const volatile uint8_t
       CUDA_TRYL(cudaEventRecord(S.ev[3], st));
       // Schur complement
       CUDA_TRYL(cudaMemsetAsync(D.S, 0, sizeof(double) * nS, st));
-      {
-        static const bool y_by_landmark = getenv("ORB_B200_LIN") && !strcmp(getenv("ORB_B200_LIN"), "landmark");
-        if (L && y_by_landmark) lm_prepare_kernel<true><<<lm_blocks, 128, 0, st>>>(D, lambda);
-        else if (L) {
-          lm_prepare_kernel<false><<<lm_blocks, 128, 0, st>>>(D, lambda);
-          y_edge_kernel<<<(E + 127) / 128, 128, 0, st>>>(D);
-          S.launches += 1;
-        }
+      if (L) {
+        lm_prepare_kernel<<<lm_blocks, 128, 0, st>>>(D, lambda);
+        y_edge_kernel<<<(E + 127) / 128, 128, 0, st>>>(D);
+        S.launches += 1;
       }
       schur_pairs_kernel<<<n_pairs, 256, 0, st>>>(D);
       bschur_kernel<<<nf, POSE_THREADS, 0, st>>>(D);
@@ -2481,17 +2326,11 @@ static int solve_impl(Solver& S, const lba_graph_view* g, const volatile uint8_t
       if (use_win) {
         const size_t smem = sizeof(double) * (WIN * WIN_P + WIN + 2 * WPB * WIN_LP + (WIN_THREADS / 32 - WIN / 32) * (WIN + 8)) +
                             sizeof(int) * ((size_t)n + (n + WPB - 1) / WPB + 4);
-        static const bool win_prof = getenv("ORB_B200_LDLT_PROF") != nullptr;
-        // ORB_B200_LDLT_FWD=thread: the forward substitution of the panel rows one thread per row (the A/B baseline
-        // of profiles/r2_summary.md) instead of on the tensor pipe through the inverse pivot block
-        static const bool fwd_thread = getenv("ORB_B200_LDLT_FWD") && !strcmp(getenv("ORB_B200_LDLT_FWD"), "thread");
-        const void* kfn = win_prof ? (fwd_thread ? (const void*)ldlt_win_kernel<true, false> : (const void*)ldlt_win_kernel<true, true>)
-                                   : (fwd_thread ? (const void*)ldlt_win_kernel<false, false> : (const void*)ldlt_win_kernel<false, true>);
+        const void* kfn = (const void*)ldlt_win_kernel;
         CUDA_TRYL(raise_dynamic_smem(kfn, smem, S.device));
-        static const int win_flags = getenv("ORB_B200_LDLT_FLAGS") ? atoi(getenv("ORB_B200_LDLT_FLAGS")) : 0;
         WinArgs wa;
         memset(&wa, 0, sizeof(wa));
-        wa.fail = D.scalars + 3; wa.flags = win_flags;
+        wa.fail = D.scalars + 3;
         void* args[] = {&wa};
         if (!use_two) {
           wa.s[0] = WinSide{D.S, d_env_reach, d_env_first, nullptr, n, 0, 0, 0};
@@ -2508,7 +2347,7 @@ static int solve_impl(Solver& S, const lba_graph_view* g, const volatile uint8_t
           sep_merge_kernel<<<ts_w + 1, 128, 0, st>>>(D.S, n, ts_m, ts_w, ts_R0, m1, ts_R1, d_dump0, d_dump1, d_Msep);
           WinArgs ws;
           memset(&ws, 0, sizeof(ws));
-          ws.fail = D.scalars + 3; ws.flags = win_flags; ws.mode = 0; ws.x = d_xs;
+          ws.fail = D.scalars + 3; ws.mode = 0; ws.x = d_xs;
           ws.s[0] = WinSide{d_Msep, d_sep_reach, d_sep_first, nullptr, ts_w, 0, 0, 0};
           void* sargs[] = {&ws};
           CUDA_TRYL(cudaLaunchKernel(kfn, dim3(1), dim3(WIN_THREADS), sargs, smem, st));
@@ -2516,7 +2355,6 @@ static int solve_impl(Solver& S, const lba_graph_view* g, const volatile uint8_t
           CUDA_TRYL(cudaLaunchKernel(kfn, dim3(2), dim3(WIN_THREADS), args, smem, st));
           S.launches += 5;
         }
-        if (win_prof) win_prof_solves++;
       } else if (use_sky) {
         const size_t smem = sizeof(double) * 2 * 32 * SKY_WMAX;
         CUDA_TRYL(raise_dynamic_smem((const void*)ldlt_sky_kernel, smem, S.device));
@@ -2527,9 +2365,7 @@ static int solve_impl(Solver& S, const lba_graph_view* g, const volatile uint8_t
         int nn = n;
         unsigned* bar = S.d_bar;
         double* failp = D.scalars + 3;
-        static const int dbg_env = getenv("ORB_B200_LDLT_DEBUG") ? atoi(getenv("ORB_B200_LDLT_DEBUG")) : 0;
-        int dbg = dbg_env;  // timing experiments only (bit0: no diagonal factor, bit1: no panel, bit2: no trailing)
-        void* args[] = {&Mp, &nn, &bar, &failp, &dbg};
+        void* args[] = {&Mp, &nn, &bar, &failp};
         const int blocks = std::min(S.ldlt_blocks, std::max(1, (n + 1 + NB - 1) / NB * ((n + 1 + NB - 1) / NB)));
         CUDA_TRYL(cudaLaunchCooperativeKernel((void*)ldlt_kernel, dim3(blocks), dim3(256), args, 0, st));
         backsub_kernel<<<1, 1024, sizeof(double) * n, st>>>(D.S, n, D.x);
@@ -2596,23 +2432,6 @@ static int solve_impl(Solver& S, const lba_graph_view* g, const volatile uint8_t
   for (int s = 0; s < E; s++) {
     if (chi2_out) chi2_out[perm[s]] = chi_sorted[s];
     if (depth_pos_out) depth_pos_out[perm[s]] = dep_sorted[s];
-  }
-  if (win_prof_solves > 0) {  // ORB_B200_LDLT_PROF: cycles per phase of ldlt_win_kernel<true>, summed over warp 0 and warp 1
-    unsigned long long pc[32] = {0}, zero[32] = {0};
-    cudaMemcpyFromSymbol(pc, g_win_prof, sizeof(pc));
-    cudaMemcpyToSymbol(g_win_prof, zero, sizeof(zero));
-    const double d = (double)win_prof_solves;
-    const char* names[8] = {"fwd-subst", "barrier A", "tiles", "barrier B", "x pass", "after fwd (row loads)", "pivot", "pivot store"};
-    for (int w = 0; w < 2; w++) {
-      fprintf(stderr, "[orbb200 lba] ldlt_win cycles per solve, warp %d (n = %d):", w, n);
-      for (int k = 0; k < 8; k++) fprintf(stderr, " %s %.0f |", names[k], pc[8 * w + k] / d);
-      fprintf(stderr, "\n");
-    }
-    const char* bn[8] = {"staging (inverse blocks)", "chain", "transform", "fetch", "barrier", "prologue", "tail barrier", "-"};
-    fprintf(stderr, "[orbb200 lba] back-substitution, thread 0:");
-    for (int k = 0; k < 7; k++) fprintf(stderr, " %s %.0f |", bn[k], pc[16 + k] / d);
-    fprintf(stderr, "\n");
-    win_prof_solves = 0;
   }
   if (stats) {
     memset(stats, 0, sizeof(*stats));

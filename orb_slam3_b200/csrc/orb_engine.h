@@ -74,7 +74,7 @@ struct Engine {
   size_t pyr_frame_bytes = 0, cand_frame_elems = 0, scratch_frame_bytes = 0, sel_frame_elems = 0;
   int out_cap = 0, num_cells = 0, num_tiles = 0, oct_smem_node_cap = 0, oct_smem_node_cap_full = 0;
   size_t oct_smem_bytes = 0;
-  int cap_rows = 0, cap_cols = 0, cap_batch = 0, cap_batch_hint = 1, chunk_override = 0;
+  int cap_rows = 0, cap_cols = 0, cap_batch = 0, cap_batch_hint = 1;
 
   // device state
   bool initialized = false;
@@ -147,7 +147,6 @@ struct Engine {
   bool resize_words_ok = false;  // resize_words_kernel (word loads + PRMT + IDP.2A) applies as well
   bool resize_rows_ok = false;  // resize_rows_kernel (shared-memory staged) applies to this pyramid geometry
   int encode_tensor_maps(int batch);
-  int l2_chunk_frames(int batch) const;
   int fetch_pyramid();
   int debug_candidates(int frame, int level, int* xys, int cap);
 };

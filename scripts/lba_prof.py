@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
-"""Phase cycle counters of ldlt_win_kernel (ORB_B200_LDLT_PROF, printed by lba_solve on stderr) for one graph.
-Usage: ORB_B200_LDLT_PROF=1 python scripts/lba_prof.py [K L]"""
+"""LocalBundleAdjustment timings (stats of the third of three solves) for one graph, as one JSON line.
+Usage: python scripts/lba_prof.py [K L]"""
 import json
 import os
 import sys
