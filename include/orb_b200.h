@@ -206,6 +206,26 @@ int match_triangulate(orb_matcher* m, const orb_frame_view* kf1, const orb_frame
                       const float* ep2, int only_stereo, int coarse, int check_orientation,
                       int32_t* pairs_out, int cap);
 
+/* int ORBmatcher(nnratio, checkOri).SearchByBoW(KeyFrame* pKF, Frame& F, vector<MapPoint*>& vpMapPointMatches)
+ * (ORBmatcher.cc:223-…), Pinhole without a second camera.  kf_mp_ok[i] (kf.n entries) = pKF->GetMapPointMatches()[i]
+ * is non-NULL and !isBad().  Reads keys[].angle and desc of both views; F.kp_taken is not read (the call starts
+ * from an all-NULL vpMapPointMatches).  fv_kf / fv_f = pKF->mFeatVec / F.mFeatVec; every feature index must occur in
+ * at most one node, as DBoW2::transform makes them.  assign_out[i] (F.n entries) = KF keypoint index whose map point
+ * lands in vpMapPointMatches[i], -1 = untouched, -2 = written and then cleared by the rotation check.
+ * Returns nmatches (the number of entries >= 0).  Malformed FeatureVectors (node ids not ascending, ptr
+ * decreasing, an index outside [0, n) or in two places) are rejected with ORB_E_ARG before any device work. */
+int match_bow_frame(orb_matcher* m, const orb_frame_view* kf, const uint8_t* kf_mp_ok, const orb_featvec_view* fv_kf,
+                    const orb_frame_view* F, const orb_featvec_view* fv_f, float nn_ratio, int check_orientation,
+                    int32_t* assign_out);
+
+/* int ORBmatcher(nnratio, checkOri).SearchByBoW(KeyFrame* pKF1, KeyFrame* pKF2, vector<MapPoint*>& vpMatches12)
+ * (ORBmatcher.cc:765-…), both Pinhole without a second camera.  mp_ok1 / mp_ok2 as kf_mp_ok above, for
+ * GetMapPointMatches() of either keyframe.  match12_out[i] (kf1.n entries) = KF2 keypoint index whose map point lands
+ * in vpMatches12[i], -1 / -2 as above.  Returns nmatches. */
+int match_bow_keyframes(orb_matcher* m, const orb_frame_view* kf1, const uint8_t* mp_ok1, const orb_featvec_view* fv1,
+                        const orb_frame_view* kf2, const uint8_t* mp_ok2, const orb_featvec_view* fv2, float nn_ratio,
+                        int check_orientation, int32_t* match12_out);
+
 /* Batched forms: `count` independent problems in one submission (frames of a
  * stream, keyframe pairs).  on_device = 0: all views are host memory.  on_device = 1: every pointer inside the
  * views (and the outputs) is a device pointer and nothing is copied.  on_device = 2 (projection matchers):
@@ -222,6 +242,20 @@ int match_triangulate_batch(orb_matcher* m, int count, const orb_frame_view* kf1
                             const orb_featvec_view* fv1, const orb_featvec_view* fv2, const float* F12_rowmajor9,
                             const float* ep2, int only_stereo, int coarse, int check_orientation,
                             int32_t* const* pairs_out, int cap, int32_t* results, int on_device);
+/* SearchByBoW batches: Relocalization (one frame against each candidate keyframe) and loop / merge detection (one
+ * keyframe pair per covisible keyframe).  Problem k reads kf_mp_ok[k] / mp_ok1[k] / mp_ok2[k] and writes
+ * assign_out[k] / match12_out[k]; results[k] = its nmatches.  on_device = 1: every array, the FeatureVectors' and the
+ * outputs included, is device memory (the FeatureVectors are then not checked: they must be well formed).
+ * on_device = 2 (match_bow_frame_batch only): the frames' keys / desc are an extractor's device results, everything
+ * else is host memory.  Repeating one frame view in several problems stages it once.  Returns count or ORB_E_*. */
+int match_bow_frame_batch(orb_matcher* m, int count, const orb_frame_view* kf, const uint8_t* const* kf_mp_ok,
+                          const orb_featvec_view* fv_kf, const orb_frame_view* F, const orb_featvec_view* fv_f,
+                          float nn_ratio, int check_orientation, int32_t* const* assign_out, int32_t* results,
+                          int on_device);
+int match_bow_keyframes_batch(orb_matcher* m, int count, const orb_frame_view* kf1, const uint8_t* const* mp_ok1,
+                              const orb_featvec_view* fv1, const orb_frame_view* kf2, const uint8_t* const* mp_ok2,
+                              const orb_featvec_view* fv2, float nn_ratio, int check_orientation,
+                              int32_t* const* match12_out, int32_t* results, int on_device);
 /* Submit subsequent batches on `cuda_stream` (a cudaStream_t) instead of the
  * matcher's own stream, e.g. the stream an extractor ran on; NULL restores it. */
 int match_set_stream(orb_matcher* m, void* cuda_stream);

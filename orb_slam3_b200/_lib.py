@@ -55,6 +55,10 @@ SIGNATURES = {
     "match_project_last_batch": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _f, _i, _vp, _vp, _i]),
     "match_project_local_batch": (_i, [_vp, _i, _vp, _vp, _f, _f, _i, _f, _vp, _vp, _i]),
     "match_triangulate_batch": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _i, _vp, _i]),
+    "match_bow_frame": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _vp]),
+    "match_bow_keyframes": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _vp]),
+    "match_bow_frame_batch": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _f, _i, _vp, _vp, _i]),
+    "match_bow_keyframes_batch": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _vp, _vp, _i]),
     "match_set_stream": (_i, [_vp, _vp]),
     "match_set_async": (_i, [_vp, _i]),
     "match_synchronize": (_i, [_vp]),

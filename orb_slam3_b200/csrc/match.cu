@@ -2,6 +2,8 @@
 //   match_project_local  <- ORBmatcher::SearchByProjection(Frame&, vector<MapPoint*>&)  ORBmatcher.cc:43-141
 //   match_project_last   <- ORBmatcher::SearchByProjection(Frame&, const Frame&)        ORBmatcher.cc:1676-1887
 //   match_triangulate    <- ORBmatcher::SearchForTriangulation                           ORBmatcher.cc:907-1146
+//   match_bow_frame      <- ORBmatcher::SearchByBoW(KeyFrame*, Frame&, vector<MapPoint*>&)     ORBmatcher.cc:223-…
+//   match_bow_keyframes  <- ORBmatcher::SearchByBoW(KeyFrame*, KeyFrame*, vector<MapPoint*>&)  ORBmatcher.cc:765-…
 //
 // The reference loops are greedy and order dependent: a keypoint already held by
 // a MapPoint with observations is skipped *before* its distance is looked at, and
@@ -554,26 +556,33 @@ __global__ void __launch_bounds__(128) tri_match_kernel(TriProblem* probs) {
   if (best >= 0 && T.check_ori) T.bins[idx1] = rot_bin(K1.keys[idx1].angle, K2.keys[best].angle);
 }
 
+// Rotation-consistency check of SearchForTriangulation and SearchByBoW, run by a whole CTA after the matching loop:
+// histogram of bins[i] over the entries with out[i] >= 0, ComputeThreeMaxima (ORBmatcher.cc:2012-2053), and every
+// such entry whose bin is not among the (at most three) maxima is set to `cleared`.  Ends with a barrier.
+__device__ void rot_filter_cta(int* out, const int* bins, int n, int cleared) {
+  __shared__ int s_hist[HISTO_LENGTH], s_ind[3];
+  for (int b = threadIdx.x; b < HISTO_LENGTH; b += blockDim.x) s_hist[b] = 0;
+  __syncthreads();
+  for (int i = threadIdx.x; i < n; i += blockDim.x)
+    if (out[i] >= 0) atomicAdd(&s_hist[bins[i]], 1);
+  __syncthreads();
+  if (threadIdx.x == 0) { int a, b, c; three_maxima(s_hist, a, b, c); s_ind[0] = a; s_ind[1] = b; s_ind[2] = c; }
+  __syncthreads();
+  for (int i = threadIdx.x; i < n; i += blockDim.x)
+    if (out[i] >= 0) {
+      const int bin = bins[i];
+      if (bin != s_ind[0] && bin != s_ind[1] && bin != s_ind[2]) out[i] = cleared;
+    }
+  __syncthreads();
+}
+
 __global__ void __launch_bounds__(1024) tri_finish_kernel(TriProblem* probs) {
-  __shared__ int s_hist[HISTO_LENGTH], s_ind[3], wsum[32], carry;
+  __shared__ int wsum[32], carry;
   TriProblem& T = probs[blockIdx.x];
   const int n = T.K1.n;
-  for (int b = threadIdx.x; b < HISTO_LENGTH; b += 1024) s_hist[b] = 0;
   if (threadIdx.x == 0) carry = 0;
   __syncthreads();
-  if (T.check_ori) {
-    for (int i = threadIdx.x; i < n; i += 1024)
-      if (T.match12[i] >= 0) atomicAdd(&s_hist[T.bins[i]], 1);
-    __syncthreads();
-    if (threadIdx.x == 0) { int a, b, c; three_maxima(s_hist, a, b, c); s_ind[0] = a; s_ind[1] = b; s_ind[2] = c; }
-    __syncthreads();
-    for (int i = threadIdx.x; i < n; i += 1024)
-      if (T.match12[i] >= 0) {
-        const int bin = T.bins[i];
-        if (bin != s_ind[0] && bin != s_ind[1] && bin != s_ind[2]) T.match12[i] = -1;
-      }
-    __syncthreads();
-  }
+  if (T.check_ori) rot_filter_cta(T.match12, T.bins, n, -1);
   // compaction in increasing idx1 (:1138-1143)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   for (int base = 0; base < n; base += 1024) {
@@ -596,6 +605,135 @@ __global__ void __launch_bounds__(1024) tri_finish_kernel(TriProblem* probs) {
     __syncthreads();
   }
   if (threadIdx.x == 0) { T.result[0] = carry; T.result[1] = carry > T.cap ? 1 : 0; }
+}
+
+// ---- SearchByBoW, both overloads (ORBmatcher.cc:223-… KeyFrame-Frame, :765-… KeyFrame-KeyFrame).
+// The query side is the (first) keyframe, the candidate side the frame / second keyframe.  Features of different
+// vocabulary nodes never compete (every feature index is in at most one node of a FeatureVector), so the shared nodes
+// are independent work items; inside a node the reference's scan is sequential over the queries, because a match takes
+// its candidate for the rest of the call.
+struct BowProblem {
+  int kind;                       // 0: SearchByBoW(KeyFrame*, Frame&)   1: SearchByBoW(KeyFrame*, KeyFrame*)
+  int nq, nc;                     // keypoints of the query side (KF / KF1) and of the candidate side (F / KF2)
+  const orb_keypoint *kq, *kc;    // angle only
+  const uint8_t *dq, *dc;
+  const uint8_t *okq, *okc;       // map point present and !isBad(); okc: kind 1 only
+  int nodes_q, nodes_c;
+  const uint32_t *nid_q, *nid_c;
+  const int *ptr_q, *idx_q, *ptr_c, *idx_c;
+  float ratio;
+  int check_ori;
+  int n_out;                      // kind 0: nc (vpMapPointMatches), kind 1: nq (vpMatches12)
+  int* out;                       // [n_out] matched index on the other side, -1 untouched, -2 cleared by the rotation check
+  int* bins;                      // [n_out] rotation bin of a match
+  uint8_t* free_c;                // [nc] candidate still available, for nodes too large for the shared-memory copy
+  int* result;                    // [1] nmatches
+};
+
+constexpr int BOW_WARPS = 4;           // one warp per shared node
+constexpr int BOW_SMEM_CAND = 256;     // candidates of a node staged in shared memory (8 KB of descriptors per warp)
+constexpr unsigned BOW_POS_BITS = 23;  // key = dist << 23 | position in the node; the host rejects n >= 2^23
+constexpr unsigned BOW_POS_MASK = (1u << BOW_POS_BITS) - 1;
+
+__global__ void __launch_bounds__(256) bow_init_kernel(const BowProblem* probs) {
+  const BowProblem& P = probs[blockIdx.x];
+  for (int i = threadIdx.x; i < P.n_out; i += 256) P.out[i] = -1;
+}
+
+// One warp per (problem, query-side node).  For each query in the node's order, lane l scans the candidates at
+// positions l, l+32, ... that are still free and keeps (min key, second-smallest distance); the butterfly merge of two
+// such pairs (a1, a2), (b1, b2) is (min(a1, b1), min(dist(max(a1, b1)), a2, b2)).  The result is the reference's
+// bestDist1 with the FIRST position reaching it (`dist < bestDist1` only moves on a strictly smaller distance) and its
+// bestDist2, the second smallest value of the distance multiset (a tie at the minimum gives bestDist2 == bestDist1).
+// Nodes up to BOW_SMEM_CAND candidates are copied to shared memory with their free flags; larger ones (levelsup >= L
+// makes the whole frame one node) read descriptors from global memory and keep the flags in P.free_c.  The scan order,
+// and hence every result, is the same on both paths.
+__global__ void __launch_bounds__(BOW_WARPS * 32) bow_match_kernel(const BowProblem* probs) {
+  __shared__ uint4 s_desc[BOW_WARPS][BOW_SMEM_CAND][2];
+  __shared__ uint8_t s_free[BOW_WARPS][BOW_SMEM_CAND];
+  const BowProblem& P = probs[blockIdx.y];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int a = blockIdx.x * BOW_WARPS + warp;
+  if (a >= P.nodes_q) return;
+  const int b = find_node(P.nid_c, P.nodes_c, P.nid_q[a]);
+  if (b < 0) return;
+  const int q0 = P.ptr_q[a], q1 = P.ptr_q[a + 1], c0 = P.ptr_c[b], m = P.ptr_c[b + 1] - c0;
+  const bool staged = m <= BOW_SMEM_CAND;
+  uint4 (*sd)[2] = s_desc[warp];
+  uint8_t* sf = s_free[warp];
+  for (int pos = lane; pos < m; pos += 32) {
+    const int idx = P.idx_c[c0 + pos];
+    const uint8_t ok = P.kind == 1 ? P.okc[idx] : 1;  // KF2: pMP2 && !isBad(); F: vpMapPointMatches starts all NULL
+    if (staged) {
+      const uint4* pd = reinterpret_cast<const uint4*>(P.dc + (size_t)idx * 32);
+      sd[pos][0] = pd[0]; sd[pos][1] = pd[1];
+      sf[pos] = ok;
+    } else {
+      P.free_c[idx] = ok;
+    }
+  }
+  __syncwarp();
+  for (int p = q0; p < q1; p++) {
+    const int i1 = P.idx_q[p];
+    if (!P.okq[i1]) continue;  // pMP && !pMP->isBad()
+    const uint4* pq = reinterpret_cast<const uint4*>(P.dq + (size_t)i1 * 32);
+    const uint4 qa = pq[0], qb = pq[1];
+    unsigned k1 = (256u << BOW_POS_BITS) | BOW_POS_MASK;  // bestDist1 = 256, no position
+    int d2 = 256;                                          // bestDist2
+    for (int pos = lane; pos < m; pos += 32) {
+      uint4 ca, cb;
+      if (staged) {
+        if (!sf[pos]) continue;
+        ca = sd[pos][0]; cb = sd[pos][1];
+      } else {
+        const int idx = P.idx_c[c0 + pos];
+        if (!P.free_c[idx]) continue;
+        const uint4* pd = reinterpret_cast<const uint4*>(P.dc + (size_t)idx * 32);
+        ca = pd[0]; cb = pd[1];
+      }
+      const int dist = __popc(qa.x ^ ca.x) + __popc(qa.y ^ ca.y) + __popc(qa.z ^ ca.z) + __popc(qa.w ^ ca.w) +
+                       __popc(qb.x ^ cb.x) + __popc(qb.y ^ cb.y) + __popc(qb.z ^ cb.z) + __popc(qb.w ^ cb.w);
+      const unsigned key = ((unsigned)dist << BOW_POS_BITS) | (unsigned)pos;
+      if (key < k1) { d2 = min(d2, (int)(k1 >> BOW_POS_BITS)); k1 = key; }
+      else d2 = min(d2, dist);
+    }
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+      const unsigned ok1 = __shfl_xor_sync(0xffffffffu, k1, o);
+      const int od2 = __shfl_xor_sync(0xffffffffu, d2, o);
+      d2 = min(min(d2, od2), (int)(max(k1, ok1) >> BOW_POS_BITS));
+      k1 = min(k1, ok1);
+    }
+    const int best = (int)(k1 >> BOW_POS_BITS);
+    // keyframe-frame accepts bestDist1 <= TH_LOW, keyframe-keyframe bestDist1 < TH_LOW
+    const bool pass = P.kind == 0 ? best <= TH_LOW : best < TH_LOW;
+    if (pass && (float)best < __fmul_rn(P.ratio, (float)d2)) {
+      const int pos = (int)(k1 & BOW_POS_MASK);
+      if (lane == 0) {
+        const int i2 = P.idx_c[c0 + pos];
+        if (staged) sf[pos] = 0; else P.free_c[i2] = 0;
+        const int r = P.kind == 0 ? i2 : i1;
+        P.out[r] = P.kind == 0 ? i1 : i2;
+        if (P.check_ori) P.bins[r] = rot_bin(P.kq[i1].angle, P.kc[i2].angle);
+      }
+    }
+    __syncwarp();  // the take is visible to every lane before the next query
+  }
+}
+
+// One CTA per problem: the rotation check over the recorded matches, then nmatches = entries still >= 0.
+__global__ void __launch_bounds__(1024) bow_finish_kernel(const BowProblem* probs) {
+  __shared__ int s_count;
+  const BowProblem& P = probs[blockIdx.x];
+  if (threadIdx.x == 0) s_count = 0;
+  __syncthreads();
+  if (P.check_ori) rot_filter_cta(P.out, P.bins, P.n_out, -2);
+  int c = 0;
+  for (int i = threadIdx.x; i < P.n_out; i += blockDim.x) c += P.out[i] >= 0;
+  c = __reduce_add_sync(0xffffffffu, c);
+  if ((threadIdx.x & 31) == 0 && c) atomicAdd(&s_count, c);
+  __syncthreads();
+  if (threadIdx.x == 0) P.result[0] = s_count;
 }
 
 // ------------------------------------------------------------------ host side
@@ -1000,6 +1138,140 @@ static int run_triangulate(Matcher& M, int count, const orb_frame_view* kf1, con
   return count;
 }
 
+// A FeatureVector over n keypoints as bow_match_kernel needs it: node ids strictly ascending, ptr non-decreasing
+// from >= 0, every index inside [0, n) and in at most one node (DBoW2::transform files each feature once).  A bad
+// index would be read out of bounds on the device, so host views are checked before anything is launched.
+static bool featvec_ok(const orb_featvec_view& f, int n, std::vector<uint8_t>& seen) {
+  if (f.n_nodes < 0) return false;
+  if (f.n_nodes == 0) return true;
+  if (!f.node_ids || !f.ptr || f.ptr[0] < 0) return false;
+  for (int k = 0; k < f.n_nodes; k++) {
+    if (f.ptr[k + 1] < f.ptr[k]) return false;
+    if (k > 0 && f.node_ids[k] <= f.node_ids[k - 1]) return false;
+  }
+  if (f.ptr[f.n_nodes] > f.ptr[0] && !f.idx) return false;
+  seen.assign(std::max(n, 0), 0);
+  for (int p = f.ptr[0]; p < f.ptr[f.n_nodes]; p++) {
+    const int i = f.idx[p];
+    if (i < 0 || i >= n || seen[i]) return false;
+    seen[i] = 1;
+  }
+  return true;
+}
+
+static bool bow_view_ok(const orb_frame_view& v, bool dev) {
+  return v.n >= 0 && v.n < (1 << BOW_POS_BITS) && (v.n == 0 || dev || (v.keys && v.desc));
+}
+
+// kind 0: q = keyframes, c = frames (on_device 2: the frames' keys / desc are an extractor's device results);
+// kind 1: q = KF1, c = KF2.  outs[k] has c[k].n (kind 0) or q[k].n (kind 1) entries.
+static int run_bow(Matcher& M, int count, int kind, const orb_frame_view* q, const uint8_t* const* okq,
+                   const orb_featvec_view* fvq, const orb_frame_view* c, const uint8_t* const* okc,
+                   const orb_featvec_view* fvc, float ratio, int check_ori, int32_t* const* outs, int32_t* results,
+                   int on_device) {
+  if (count <= 0 || !q || !okq || !fvq || !c || !fvc || (kind == 1 && !okc) || !outs || !results ||
+      on_device < 0 || on_device > (kind == 0 ? 2 : 1)) {
+    set_last_error("bad argument");
+    return ORB_E_ARG;
+  }
+  const bool all_dev = on_device == 1;
+  std::vector<uint8_t> seen;
+  for (int k = 0; k < count; k++) {
+    if (!bow_view_ok(q[k], all_dev) || !bow_view_ok(c[k], on_device != 0) || !outs[k] ||
+        (q[k].n > 0 && !okq[k]) || (kind == 1 && c[k].n > 0 && !okc[k])) {
+      set_last_error("bad argument: view, map point flags or output");
+      return ORB_E_ARG;
+    }
+    if (!all_dev && (!featvec_ok(fvq[k], q[k].n, seen) || !featvec_ok(fvc[k], c[k].n, seen))) {
+      set_last_error("malformed FeatureVector: node ids must ascend, ptr must not decrease, every index must lie in "
+                     "[0, n) and occur once");
+      return ORB_E_ARG;
+    }
+  }
+  int rc = M.init();
+  if (rc) return rc;
+  CUDA_TRYM(cudaSetDevice(M.device));
+  if ((rc = M.finish_pending())) return rc;
+  std::vector<BowProblem> P(count);
+  Stager st{all_dev};
+  for (int pass = 0; pass < 2; pass++) {
+    st.off = 0;
+    for (int k = 0; k < count; k++) {
+      BowProblem& p = P[k];
+      memset(&p, 0, sizeof(p));
+      p.kind = kind;
+      p.nq = q[k].n; p.nc = c[k].n;
+      p.kq = st.put(q[k].keys, q[k].n); p.dq = st.put(q[k].desc, (size_t)q[k].n * 32);
+      p.okq = st.put(okq[k], q[k].n);
+      if (on_device == 2) {
+        p.kc = c[k].keys; p.dc = c[k].desc;
+      } else {  // Relocalization matches one frame against many keyframes: the frame is staged once
+        int j = 0;
+        while (j < k && !(c[j].keys == c[k].keys && c[j].desc == c[k].desc && c[j].n == c[k].n)) j++;
+        if (j < k) { p.kc = P[j].kc; p.dc = P[j].dc; }
+        else { p.kc = st.put(c[k].keys, c[k].n); p.dc = st.put(c[k].desc, (size_t)c[k].n * 32); }
+      }
+      if (kind == 1) p.okc = st.put(okc[k], c[k].n);
+      // device views (on_device 1): the CSR arrays are the caller's device memory; only n_nodes is read here
+      p.nodes_q = fvq[k].n_nodes; p.nodes_c = fvc[k].n_nodes;
+      const size_t fq = (all_dev || !fvq[k].n_nodes) ? 0 : (size_t)fvq[k].ptr[fvq[k].n_nodes];
+      const size_t fc = (all_dev || !fvc[k].n_nodes) ? 0 : (size_t)fvc[k].ptr[fvc[k].n_nodes];
+      p.nid_q = st.put(fvq[k].node_ids, fvq[k].n_nodes); p.nid_c = st.put(fvc[k].node_ids, fvc[k].n_nodes);
+      p.ptr_q = st.put(fvq[k].ptr, fvq[k].n_nodes + 1); p.ptr_c = st.put(fvc[k].ptr, fvc[k].n_nodes + 1);
+      p.idx_q = st.put(fvq[k].idx, fq); p.idx_c = st.put(fvc[k].idx, fc);
+      p.ratio = ratio; p.check_ori = check_ori;
+      p.n_out = kind == 0 ? c[k].n : q[k].n;
+    }
+    if (pass == 0) {
+      if (M.h_in.reserve(std::max<size_t>(st.off, 16))) return ORB_E_CUDA;
+      if (M.in_arena.reserve(std::max<size_t>(st.off, 16))) return ORB_E_CUDA;
+      st.h_base = M.h_in.h;
+      st.d_base = M.in_arena.d;
+    }
+  }
+  const size_t in_bytes = st.off;
+  size_t sbytes = sizeof(BowProblem) * count + 4096, obytes = 0;
+  for (int k = 0; k < count; k++) {
+    sbytes += 512 + (size_t)P[k].n_out * 4 + (size_t)P[k].nc;
+    obytes += 512 + (all_dev ? 0 : (size_t)P[k].n_out * 4);
+  }
+  if (M.scratch.reserve(sbytes) || M.out_arena.reserve(obytes) || M.h_out.reserve(obytes)) return ORB_E_CUDA;
+  M.scratch.used = 0; M.out_arena.used = 0;
+  BowProblem* d_probs = carve_dev<BowProblem>(M.scratch, count);
+  int max_nodes = 0;
+  std::vector<size_t> res_off(count), out_off(count);
+  for (int k = 0; k < count; k++) {
+    BowProblem& p = P[k];
+    max_nodes = std::max(max_nodes, p.nodes_q);
+    p.bins = carve_dev<int>(M.scratch, p.n_out);
+    p.free_c = carve_dev<uint8_t>(M.scratch, p.nc);
+    res_off[k] = M.out_arena.used;
+    p.result = carve_dev<int>(M.out_arena, 1);
+    if (all_dev) p.out = outs[k];
+    else { out_off[k] = M.out_arena.used; p.out = carve_dev<int>(M.out_arena, p.n_out); }
+  }
+  cudaStream_t s = M.user_stream ? M.user_stream : M.stream;
+  CUDA_TRYM(cudaEventRecord(M.ev0, s));
+  if (in_bytes) CUDA_TRYM(cudaMemcpyAsync(M.in_arena.d, M.h_in.h, in_bytes, cudaMemcpyHostToDevice, s));
+  CUDA_TRYM(cudaMemcpyAsync(d_probs, P.data(), sizeof(BowProblem) * count, cudaMemcpyHostToDevice, s));
+  bow_init_kernel<<<count, 256, 0, s>>>(d_probs);
+  if (max_nodes > 0) bow_match_kernel<<<dim3((max_nodes + BOW_WARPS - 1) / BOW_WARPS, count), BOW_WARPS * 32, 0, s>>>(d_probs);
+  bow_finish_kernel<<<count, 1024, 0, s>>>(d_probs);
+  M.launches += 2 + (max_nodes > 0);
+  CUDA_TRYM(cudaGetLastError());
+  CUDA_TRYM(cudaMemcpyAsync(M.h_out.h, M.out_arena.d, M.out_arena.used, cudaMemcpyDeviceToHost, s));
+  CUDA_TRYM(cudaEventRecord(M.ev1, s));
+  CUDA_TRYM(cudaStreamSynchronize(s));
+  float ms = 0;
+  cudaEventElapsedTime(&ms, M.ev0, M.ev1);
+  M.last_ms = ms;
+  for (int k = 0; k < count; k++) {
+    results[k] = *(const int*)(M.h_out.h + res_off[k]);
+    if (!all_dev && P[k].n_out) memcpy(outs[k], M.h_out.h + out_off[k], sizeof(int) * (size_t)P[k].n_out);
+  }
+  return count;
+}
+
 }  // namespace orbb200
 
 using orbb200::Matcher;
@@ -1082,6 +1354,47 @@ int match_triangulate_batch(orb_matcher* m, int count, const orb_frame_view* kf1
   if (!m) return ORB_E_ARG;
   return orbb200::run_triangulate(m->m, count, kf1, kf2, fv1, fv2, F12_rowmajor9, ep2, only_stereo, coarse,
                                   check_orientation, pairs_out, cap, results, on_device);
+}
+
+int match_bow_frame(orb_matcher* m, const orb_frame_view* kf, const uint8_t* kf_mp_ok, const orb_featvec_view* fv_kf,
+                    const orb_frame_view* F, const orb_featvec_view* fv_f, float nn_ratio, int check_orientation,
+                    int32_t* assign_out) {
+  if (!m) return ORB_E_ARG;
+  int32_t res = 0;
+  int32_t* outs[1] = {assign_out};
+  const uint8_t* ok[1] = {kf_mp_ok};
+  int rc = orbb200::run_bow(m->m, 1, 0, kf, ok, fv_kf, F, nullptr, fv_f, nn_ratio, check_orientation, outs, &res, 0);
+  return rc < 0 ? rc : res;
+}
+
+int match_bow_keyframes(orb_matcher* m, const orb_frame_view* kf1, const uint8_t* mp_ok1, const orb_featvec_view* fv1,
+                        const orb_frame_view* kf2, const uint8_t* mp_ok2, const orb_featvec_view* fv2, float nn_ratio,
+                        int check_orientation, int32_t* match12_out) {
+  if (!m) return ORB_E_ARG;
+  int32_t res = 0;
+  int32_t* outs[1] = {match12_out};
+  const uint8_t* ok1[1] = {mp_ok1};
+  const uint8_t* ok2[1] = {mp_ok2};
+  int rc = orbb200::run_bow(m->m, 1, 1, kf1, ok1, fv1, kf2, ok2, fv2, nn_ratio, check_orientation, outs, &res, 0);
+  return rc < 0 ? rc : res;
+}
+
+int match_bow_frame_batch(orb_matcher* m, int count, const orb_frame_view* kf, const uint8_t* const* kf_mp_ok,
+                          const orb_featvec_view* fv_kf, const orb_frame_view* F, const orb_featvec_view* fv_f,
+                          float nn_ratio, int check_orientation, int32_t* const* assign_out, int32_t* results,
+                          int on_device) {
+  if (!m) return ORB_E_ARG;
+  return orbb200::run_bow(m->m, count, 0, kf, kf_mp_ok, fv_kf, F, nullptr, fv_f, nn_ratio, check_orientation,
+                          assign_out, results, on_device);
+}
+
+int match_bow_keyframes_batch(orb_matcher* m, int count, const orb_frame_view* kf1, const uint8_t* const* mp_ok1,
+                              const orb_featvec_view* fv1, const orb_frame_view* kf2, const uint8_t* const* mp_ok2,
+                              const orb_featvec_view* fv2, float nn_ratio, int check_orientation,
+                              int32_t* const* match12_out, int32_t* results, int on_device) {
+  if (!m) return ORB_E_ARG;
+  return orbb200::run_bow(m->m, count, 1, kf1, mp_ok1, fv1, kf2, mp_ok2, fv2, nn_ratio, check_orientation,
+                          match12_out, results, on_device);
 }
 
 int match_set_stream(orb_matcher* m, void* cuda_stream) {

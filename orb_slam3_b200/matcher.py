@@ -1,5 +1,5 @@
 """Host-side mirror of ORB_SLAM3::ORBmatcher (include/ORBmatcher.h:43-76) for the
-three hot-path methods, over the C ABI.  Frames/KeyFrames/MapPoints are passed
+hot-path methods, over the C ABI.  Frames/KeyFrames/MapPoints are passed
 as the flat views of views.py.  No CPU fallback."""
 import ctypes as C
 
@@ -61,6 +61,26 @@ class ORBmatcher:
                                               int(self.mbCheckOrientation), ptr(out), cap))
         return n, out[:n]
 
+    def SearchByBoW(self, pKF, kf_mp_ok, fv_kf, F, fv_f):
+        """SearchByBoW(KeyFrame* pKF, Frame& F, vpMapPointMatches): (nmatches, assign[F.n]); assign = KF keypoint
+        index whose map point lands in vpMapPointMatches[i], -1 untouched, -2 cleared by the rotation check.
+        kf_mp_ok[i] = the KF's map point i exists and is not bad."""
+        ok = np.ascontiguousarray(kf_mp_ok, np.uint8)
+        out = np.empty(F.n, np.int32)
+        n = check(self._lib.match_bow_frame(self._h, C.byref(pKF), ptr(ok), C.byref(fv_kf), C.byref(F), C.byref(fv_f),
+                                            self.mfNNratio, int(self.mbCheckOrientation), ptr(out)))
+        return n, out
+
+    def SearchByBoWKeyFrames(self, pKF1, mp_ok1, fv1, pKF2, mp_ok2, fv2):
+        """SearchByBoW(KeyFrame* pKF1, KeyFrame* pKF2, vpMatches12): (nmatches, match12[pKF1.n]); match12 = KF2
+        keypoint index, -1 untouched, -2 cleared by the rotation check."""
+        ok1 = np.ascontiguousarray(mp_ok1, np.uint8)
+        ok2 = np.ascontiguousarray(mp_ok2, np.uint8)
+        out = np.empty(pKF1.n, np.int32)
+        n = check(self._lib.match_bow_keyframes(self._h, C.byref(pKF1), ptr(ok1), C.byref(fv1), C.byref(pKF2), ptr(ok2),
+                                                C.byref(fv2), self.mfNNratio, int(self.mbCheckOrientation), ptr(out)))
+        return n, out
+
     # ---- batched submissions (independent problems)
     def project_last_batch(self, curs, lasts, Tcw, th, forward=None, backward=None, on_device=False,
                            assign_ptrs=None):
@@ -116,6 +136,48 @@ class ORBmatcher:
         check(self._lib.match_triangulate_batch(self._h, B, a1, a2, f1, f2, ptr(F), ptr(e), int(bOnlyStereo),
                                                 int(bCoarse), int(self.mbCheckOrientation), arr, cap, ptr(res), 0))
         return res, [o[:r] for o, r in zip(outs, res)]
+
+    def bow_frame_batch(self, kfs, kf_mp_oks, fv_kfs, frames, fv_fs, on_device=0, out_ptrs=None):
+        """SearchByBoW(KeyFrame*, Frame&) for each (kfs[k], frames[k]).  on_device = 2: the frame views' keys / desc
+        are an extractor's device results; 1: every array is device memory and out_ptrs are device outputs.
+        Returns (nmatches[B], assign lists or None)."""
+        from .views import orb_frame_view, orb_featvec_view
+        B = len(kfs)
+        oks = [np.ascontiguousarray(o, np.uint8) for o in kf_mp_oks] if int(on_device) != 1 else None
+        ok_arr = (C.c_void_p * B)(*([o.ctypes.data for o in oks] if oks is not None else kf_mp_oks))
+        res = np.zeros(B, np.int32)
+        if int(on_device) == 1:
+            outs = None
+            arr = (C.c_void_p * B)(*out_ptrs)
+        else:
+            outs = [np.empty(f.n, np.int32) for f in frames]
+            arr = (C.c_void_p * B)(*[o.ctypes.data for o in outs])
+        check(self._lib.match_bow_frame_batch(self._h, B, (orb_frame_view * B)(*kfs), ok_arr,
+                                              (orb_featvec_view * B)(*fv_kfs), (orb_frame_view * B)(*frames),
+                                              (orb_featvec_view * B)(*fv_fs), self.mfNNratio,
+                                              int(self.mbCheckOrientation), arr, ptr(res), int(on_device)))
+        return res, outs
+
+    def bow_keyframes_batch(self, kf1s, mp_ok1s, fv1s, kf2s, mp_ok2s, fv2s, on_device=0, out_ptrs=None):
+        """SearchByBoW(KeyFrame*, KeyFrame*) for each pair.  Returns (nmatches[B], match12 lists or None)."""
+        from .views import orb_frame_view, orb_featvec_view
+        B = len(kf1s)
+        dev = int(on_device) == 1
+        keep = [] if dev else [np.ascontiguousarray(o, np.uint8) for o in list(mp_ok1s) + list(mp_ok2s)]
+        p1 = list(mp_ok1s) if dev else [o.ctypes.data for o in keep[:B]]
+        p2 = list(mp_ok2s) if dev else [o.ctypes.data for o in keep[B:]]
+        res = np.zeros(B, np.int32)
+        if dev:
+            outs = None
+            arr = (C.c_void_p * B)(*out_ptrs)
+        else:
+            outs = [np.empty(k.n, np.int32) for k in kf1s]
+            arr = (C.c_void_p * B)(*[o.ctypes.data for o in outs])
+        check(self._lib.match_bow_keyframes_batch(self._h, B, (orb_frame_view * B)(*kf1s), (C.c_void_p * B)(*p1),
+                                                  (orb_featvec_view * B)(*fv1s), (orb_frame_view * B)(*kf2s),
+                                                  (C.c_void_p * B)(*p2), (orb_featvec_view * B)(*fv2s), self.mfNNratio,
+                                                  int(self.mbCheckOrientation), arr, ptr(res), int(on_device)))
+        return res, outs
 
     def set_stream(self, cuda_stream):
         check(self._lib.match_set_stream(self._h, C.c_void_p(cuda_stream) if cuda_stream else None))

@@ -119,6 +119,71 @@ def triangulation_scene(kps1, desc1, kps2, desc2, width, height, seed, n_nodes=1
     return k1, k2, make_featvec_view(node1), make_featvec_view(node2), F12.reshape(9), ep
 
 
+def hash_nodes(desc, n_nodes=1000):
+    """A FeatureVector stand-in without a vocabulary: node of a feature = a hash of its first two descriptor bytes."""
+    w = np.asarray(desc)[:, :2].astype(np.int64)
+    return ((w[:, 0] >> 3) * 32 + (w[:, 1] >> 3)) % n_nodes
+
+
+def nodes_from_featvec(n, fv_node_ids, fv_ptr, fv_idx):
+    """Per-feature node id (-1 = not in the vector) of a FeatureVector CSR, e.g. the output of bow_transform."""
+    node = -np.ones(n, np.int64)
+    for k, nid in enumerate(fv_node_ids):
+        node[fv_idx[fv_ptr[k]:fv_ptr[k + 1]]] = int(nid)
+    return node
+
+
+def bow_match_scene(n, seed, node_of, width=1280, height=720, bad_frac=0.3, dup_frac=0.1, outlier_frac=0.15,
+                    max_flip=60):
+    """SearchByBoW: two views of one set of n keypoints.  View 2 holds a permuted (1 - dup_frac - outlier_frac) share
+    of view 1's keypoints with each descriptor perturbed by 0..max_flip flipped bits, dup_frac second copies of some
+    of them (near ties for the ratio test), and outlier_frac gross outliers (random descriptors).  Its angles are view
+    1's minus an offset drawn around 0, 30, 75, 200 and 355 degrees, so the matches fill several rotation bins.
+    bad_frac of the map points of either side are missing or bad.  node_of(desc) -> node id per feature (-1 = not in
+    the FeatureVector), e.g. the vocabulary descent of DBoW2::transform at some levelsup, or hash_nodes.
+    Returns dict(kf1, ok1, fv1, kf2, ok2, fv2): view 1 is the keyframe (query side), view 2 the frame or second
+    keyframe."""
+    from ._lib import KP_DTYPE
+    rng = np.random.default_rng(seed)
+    sf = scale_factors()
+
+    def keypoints(x, y, angle, octave):
+        k = np.zeros(len(x), KP_DTYPE)
+        k["x"], k["y"], k["angle"], k["octave"] = x, y, angle, octave
+        k["size"] = 31.0 * sf[octave]
+        k["response"] = rng.uniform(10, 100, len(x))
+        k["class_id"] = -1
+        return k
+
+    ang1 = rng.uniform(0, 360, n).astype(np.float32)
+    oct1 = rng.integers(0, 8, n)
+    k1 = keypoints(rng.uniform(20, width - 20, n), rng.uniform(20, height - 20, n), ang1, oct1)
+    d1 = rng.integers(0, 256, (n, 32), dtype=np.uint8)
+    n_dup, n_out = int(dup_frac * n), int(outlier_frac * n)
+    base = rng.permutation(n)[:n - n_dup - n_out]
+    rows = np.concatenate([base, rng.choice(base, n_dup)]) if len(base) else base
+    d2 = d1[rows].copy()
+    for i, k in enumerate(rng.integers(0, max_flip + 1, len(rows))):
+        bits = np.unpackbits(d2[i])
+        bits[rng.choice(256, k, replace=False)] ^= 1
+        d2[i] = np.packbits(bits)
+    d2 = np.concatenate([d2, rng.integers(0, 256, (n_out, 32), dtype=np.uint8)])
+    offset = rng.choice([0.0, 30.0, 75.0, 200.0, 355.0], len(rows), p=[0.4, 0.2, 0.15, 0.1, 0.15])
+    ang2 = np.mod(ang1[rows] - offset - rng.uniform(-8, 8, len(rows)), 360.0)
+    ang2 = np.concatenate([ang2, rng.uniform(0, 360, n_out)]).astype(np.float32)
+    ang2[ang2 >= 360.0] = 0.0
+    x2 = np.concatenate([k1["x"][rows] + rng.normal(0, 2, len(rows)), rng.uniform(20, width - 20, n_out)])
+    y2 = np.concatenate([k1["y"][rows] + rng.normal(0, 2, len(rows)), rng.uniform(20, height - 20, n_out)])
+    oct2 = np.concatenate([oct1[rows], rng.integers(0, 8, n_out)])
+    order = rng.permutation(len(d2))
+    k2 = keypoints(x2[order], y2[order], ang2[order], oct2[order])
+    d2 = np.ascontiguousarray(d2[order])
+    kf1 = make_frame_view(k1, d1, width, height, sf, fx=FX, fy=FY)
+    kf2 = make_frame_view(k2, d2, width, height, sf, fx=FX, fy=FY)
+    return dict(kf1=kf1, ok1=(rng.random(n) >= bad_frac).astype(np.uint8), fv1=make_featvec_view(node_of(d1)),
+                kf2=kf2, ok2=(rng.random(len(d2)) >= bad_frac).astype(np.uint8), fv2=make_featvec_view(node_of(d2)))
+
+
 # ---------------------------------------------------------------- local BA graphs
 def _quat_from_yaw_pitch(yaw, pitch):
     cy, sy, cp, sp = np.cos(yaw / 2), np.sin(yaw / 2), np.cos(pitch / 2), np.sin(pitch / 2)

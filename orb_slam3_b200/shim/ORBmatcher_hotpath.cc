@@ -1,4 +1,4 @@
-// Replacements for three ORBmatcher methods (reference src/ORBmatcher.cc) that
+// Replacements for the hot-path ORBmatcher methods (reference src/ORBmatcher.cc) that
 // flatten Frame / KeyFrame / MapPoint state into the views of orb_b200.h and
 // forward to liborbb200.so.  Build inside the ORB_SLAM3 tree: delete the bodies
 // of these methods from src/ORBmatcher.cc (or compile that file with
@@ -61,6 +61,29 @@ void frame_view(Frame& F, FrameArrays& a) {
   fill_common(F, F.mvKeysUn, F.mvuRight, F.mDescriptors, a);
   a.v.min_x = Frame::mnMinX; a.v.min_y = Frame::mnMinY; a.v.max_x = Frame::mnMaxX; a.v.max_y = Frame::mnMaxY;
   a.v.grid_w_inv = Frame::mfGridElementWidthInv; a.v.grid_h_inv = Frame::mfGridElementHeightInv;
+}
+
+struct FeatVecArrays {  // DBoW2::FeatureVector as the CSR of orb_featvec_view
+  std::vector<uint32_t> ids;
+  std::vector<int32_t> ptr, idx;
+  orb_featvec_view v;
+};
+
+void featvec_view(const DBoW2::FeatureVector& fv, FeatVecArrays& a) {
+  a.ptr.push_back(0);
+  for (const auto& kv : fv) {  // std::map: ascending node id
+    a.ids.push_back(kv.first);
+    for (unsigned int i : kv.second) a.idx.push_back((int32_t)i);
+    a.ptr.push_back((int32_t)a.idx.size());
+  }
+  a.v = orb_featvec_view{(int32_t)a.ids.size(), a.ids.data(), a.ptr.data(), a.idx.data()};
+}
+
+// pMP && !pMP->isBad() for every entry of one GetMapPointMatches() snapshot
+std::vector<uint8_t> mappoint_ok(const std::vector<MapPoint*>& mps) {
+  std::vector<uint8_t> ok(mps.size(), 0);
+  for (size_t i = 0; i < mps.size(); i++) ok[i] = mps[i] && !mps[i]->isBad();
+  return ok;
 }
 
 }  // namespace
@@ -145,24 +168,12 @@ int ORBmatcher::SearchForTriangulation(KeyFrame* pKF1, KeyFrame* pKF2, vector<pa
       if (kf->GetMapPoint(i)) a.taken[i] = 1;  // :972-977, :1003-1005
     fill_common(*kf, kf->mvKeysUn, kf->mvuRight, kf->mDescriptors, a);
   };
-  auto featvec = [](const DBoW2::FeatureVector& fv, std::vector<uint32_t>& ids, std::vector<int32_t>& ptr,
-                    std::vector<int32_t>& idx, orb_featvec_view& v) {
-    ptr.push_back(0);
-    for (const auto& kv : fv) {  // std::map: ascending node id
-      ids.push_back(kv.first);
-      for (unsigned int i : kv.second) idx.push_back((int32_t)i);
-      ptr.push_back((int32_t)idx.size());
-    }
-    v = orb_featvec_view{(int32_t)ids.size(), ids.data(), ptr.data(), idx.data()};
-  };
   FrameArrays a1, a2;
   kf_view(pKF1, a1);
   kf_view(pKF2, a2);
-  std::vector<uint32_t> id1, id2;
-  std::vector<int32_t> p1, p2, i1, i2;
-  orb_featvec_view f1, f2;
-  featvec(pKF1->mFeatVec, id1, p1, i1, f1);
-  featvec(pKF2->mFeatVec, id2, p2, i2, f2);
+  FeatVecArrays f1, f2;
+  featvec_view(pKF1->mFeatVec, f1);
+  featvec_view(pKF2->mFeatVec, f2);
   // epipole and fundamental matrix exactly as the reference computes them (:914-920, Pinhole.cpp:107-112)
   const Sophus::SE3f T1w = pKF1->GetPose(), T2w = pKF2->GetPose(), Tw2 = pKF2->GetPoseInverse();
   const Eigen::Vector2f ep = pKF2->mpCamera->project(T2w * pKF1->GetCameraCenter());
@@ -175,13 +186,58 @@ int ORBmatcher::SearchForTriangulation(KeyFrame* pKF1, KeyFrame* pKF2, vector<pa
     for (int c = 0; c < 3; c++) Frm[3 * r + c] = F12(r, c);
   const float epv[2] = {ep(0), ep(1)};
   std::vector<int32_t> pairs(2 * (size_t)pKF1->N + 2);
-  const int n = match_triangulate(matcher_for_this_thread(), &a1.v, &a2.v, &f1, &f2, Frm, epv, bOnlyStereo, bCoarse,
+  const int n = match_triangulate(matcher_for_this_thread(), &a1.v, &a2.v, &f1.v, &f2.v, Frm, epv, bOnlyStereo, bCoarse,
                                   mbCheckOrientation, pairs.data(), pKF1->N + 1);
   if (n < 0) throw std::runtime_error(orb_last_error());
   vMatchedPairs.clear();
   vMatchedPairs.reserve(n);
   for (int i = 0; i < n; i++) vMatchedPairs.push_back(make_pair((size_t)pairs[2 * i], (size_t)pairs[2 * i + 1]));
   return n;
+}
+
+// ORBmatcher.cc:223-…  (Tracking::TrackReferenceKeyFrame, Tracking::Relocalization)
+int ORBmatcher::SearchByBoW(KeyFrame* pKF, Frame& F, vector<MapPoint*>& vpMapPointMatches) {
+  if (!orbb200_gate::gpu_path(pKF) || !orbb200_gate::gpu_path(F))
+    return SearchByBoW_Reference(pKF, F, vpMapPointMatches);
+  const vector<MapPoint*> vpMapPointsKF = pKF->GetMapPointMatches();  // one snapshot: flags and write-back agree
+  const std::vector<uint8_t> ok = mappoint_ok(vpMapPointsKF);
+  vpMapPointMatches = vector<MapPoint*>(F.N, static_cast<MapPoint*>(NULL));
+  FrameArrays ka, fa;
+  fill_common(*pKF, pKF->mvKeysUn, pKF->mvuRight, pKF->mDescriptors, ka);
+  fill_common(F, F.mvKeysUn, F.mvuRight, F.mDescriptors, fa);
+  FeatVecArrays fk, ff;
+  featvec_view(pKF->mFeatVec, fk);
+  featvec_view(F.mFeatVec, ff);
+  std::vector<int32_t> assign(F.N);
+  const int nmatches = match_bow_frame(matcher_for_this_thread(), &ka.v, ok.data(), &fk.v, &fa.v, &ff.v, mfNNratio,
+                                       mbCheckOrientation, assign.data());
+  if (nmatches < 0) throw std::runtime_error(orb_last_error());
+  for (int i = 0; i < F.N; i++)
+    if (assign[i] >= 0) vpMapPointMatches[i] = vpMapPointsKF[assign[i]];  // -2: cleared by the rotation check
+  return nmatches;
+}
+
+// ORBmatcher.cc:765-…  (LoopClosing: loop and merge detection)
+int ORBmatcher::SearchByBoW(KeyFrame* pKF1, KeyFrame* pKF2, vector<MapPoint*>& vpMatches12) {
+  if (!orbb200_gate::gpu_path(pKF1) || !orbb200_gate::gpu_path(pKF2))
+    return SearchByBoW_Reference(pKF1, pKF2, vpMatches12);
+  const vector<MapPoint*> vpMapPoints1 = pKF1->GetMapPointMatches();
+  const vector<MapPoint*> vpMapPoints2 = pKF2->GetMapPointMatches();
+  const std::vector<uint8_t> ok1 = mappoint_ok(vpMapPoints1), ok2 = mappoint_ok(vpMapPoints2);
+  vpMatches12 = vector<MapPoint*>(vpMapPoints1.size(), static_cast<MapPoint*>(NULL));
+  FrameArrays a1, a2;
+  fill_common(*pKF1, pKF1->mvKeysUn, pKF1->mvuRight, pKF1->mDescriptors, a1);
+  fill_common(*pKF2, pKF2->mvKeysUn, pKF2->mvuRight, pKF2->mDescriptors, a2);
+  FeatVecArrays f1, f2;
+  featvec_view(pKF1->mFeatVec, f1);
+  featvec_view(pKF2->mFeatVec, f2);
+  std::vector<int32_t> match12(pKF1->N);
+  const int nmatches = match_bow_keyframes(matcher_for_this_thread(), &a1.v, ok1.data(), &f1.v, &a2.v, ok2.data(),
+                                           &f2.v, mfNNratio, mbCheckOrientation, match12.data());
+  if (nmatches < 0) throw std::runtime_error(orb_last_error());
+  for (int i = 0; i < pKF1->N; i++)
+    if (match12[i] >= 0) vpMatches12[i] = vpMapPoints2[match12[i]];
+  return nmatches;
 }
 
 }  // namespace ORB_SLAM3

@@ -44,6 +44,12 @@ def main(ref, out):
     t = patch(t, r"int SearchForTriangulation\(KeyFrame \*pKF1, KeyFrame\* pKF2,\s*std::vector<pair<size_t, size_t> > &vMatchedPairs, const bool bOnlyStereo, const bool bCoarse[^;]*;",
               "    int SearchForTriangulation_Reference(KeyFrame *pKF1, KeyFrame* pKF2, std::vector<pair<size_t, size_t> > &vMatchedPairs, const bool bOnlyStereo, const bool bCoarse);",
               "SearchForTriangulation_Reference")
+    t = patch(t, r"int SearchByBoW\(KeyFrame\s*\*\s*pKF,\s*Frame\s*&\s*F,[^;]*;",
+              "    int SearchByBoW_Reference(KeyFrame *pKF, Frame &F, std::vector<MapPoint*> &vpMapPointMatches);",
+              "SearchByBoW_Reference (keyframe-frame)")
+    t = patch(t, r"int SearchByBoW\(KeyFrame\s*\*\s*pKF1,\s*KeyFrame\s*\*\s*pKF2,[^;]*;",
+              "    int SearchByBoW_Reference(KeyFrame *pKF1, KeyFrame* pKF2, std::vector<MapPoint*> &vpMatches12);",
+              "SearchByBoW_Reference (keyframe-keyframe)")
     open(P("ORBmatcher.h"), "w").write(t)
 
     t = open(P("Tracking.h")).read()
